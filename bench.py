@@ -2,7 +2,7 @@
 """bench.py — rays/sec and grid-voxels/sec of the NeRF render / mesh hot path on N B200s (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload lego|fern|buff|mesh] [--shard auto|replica|rows] [--only]
+                    [--workload lego|fern|buff|mesh] [--shard auto|replica|rows] [--only] [--dump-outputs DIR]
 
 Workloads (BASELINE.json configs[1..4], SURVEY 8d; weights of the reference's shipped checkpoints re-packed under
 tests/golden/, synthetic poses, no dataset or network needed):
@@ -296,8 +296,9 @@ def make_model(nm, name, ctx, precision):
     return model, eng
 
 
-def run_render(nm, name, ctx, steps, warmup, precision, with_e2e, clocks=None):
-    """Device-resident (pose in, maps out) timing of one render workload, optionally followed by the host-buffer arm."""
+def run_render(nm, name, ctx, steps, warmup, precision, with_e2e, clocks=None, keep=False):
+    """Device-resident (pose in, maps out) timing of one render workload, optionally followed by the host-buffer arm.
+    keep: also return the maps of the last timed step, copied to the host (res["outputs"])."""
     from nerfmeshes_b200 import parallel as par
     wl = WORKLOADS[name]
     model, eng = make_model(nm, name, ctx, precision)
@@ -333,6 +334,8 @@ def run_render(nm, name, ctx, steps, warmup, precision, with_e2e, clocks=None):
     images = steps * (1 if rows else ctx.world)
     res = dict(dev_ms=dev_ms, launches=int(launches), mlp_ms=mlp_ms, mlp_pts=mlp_pts, mlp_n=mlp_n, clk=clk, finite=finite,
                rays=H * W * images)
+    if keep:        # copied now: with --shard rows the maps are views of the exchange buffers the e2e arm reuses
+        res["outputs"] = {k: v.cpu() for k, v in out.items()}
 
     if wl["buff"]:          # the AABB sampler alone (a10): warp per ray x 1533 voxels + two bitonic sorts
         o_d, d_d = eng.ray_bundle(pose_of(0), H, W, focal)
@@ -395,9 +398,10 @@ def run_render(nm, name, ctx, steps, warmup, precision, with_e2e, clocks=None):
     return res
 
 
-def run_mesh(nm, ctx, steps, warmup, precision):
+def run_mesh(nm, ctx, steps, warmup, precision, keep=False):
     """512^3 sigma sweep -> adaptive iso -> marching cubes [-> all_gather of the slab meshes]; everything inside the timed
-    region, x-slabs across ranks.  Returns per-stage times (max over ranks is taken by the caller)."""
+    region, x-slabs across ranks.  Returns per-stage times (max over ranks is taken by the caller); keep: also the mesh of
+    the last timed step, copied to the host (res["outputs"])."""
     from nerfmeshes_b200 import parallel as par
     model, eng = make_model(nm, "lego", ctx, precision)
 
@@ -421,6 +425,8 @@ def run_mesh(nm, ctx, steps, warmup, precision):
     ctx.barrier()
     res = dict(total_ms=e0.elapsed_time(e1) / steps, launches=(eng.launch_count() - l0) // steps, n_vertices=int(v.shape[0]),
                n_triangles=int(f.shape[0]), iso=float(iso), **{k: acc[k] / steps for k in keys})
+    if keep:
+        res["outputs"] = {"vertices": v.cpu(), "faces": f.cpu(), "normals": n.cpu(), "iso": torch.tensor(float(iso))}
     del model, eng, v, f, n
     torch.cuda.empty_cache()
     return res
@@ -453,6 +459,26 @@ def run_train(nm, ctx, precision):
     return res
 
 
+DUMP_BYTES = 60 << 20          # under 64 MB (decimal) with the .npy headers
+
+
+def dump_outputs(path, arrays):
+    """Write each array as <path>/<name>.npy, in float32 (float64 stays float64; integer arrays become float64, which
+    holds them exactly).  Above DUMP_BYTES in all, every array keeps the same fraction of its rows, picked by a fixed seed,
+    so two runs with the same arguments write the same rows."""
+    os.makedirs(path, exist_ok=True)
+    arrs = {}
+    for k, v in arrays.items():
+        a = v.numpy()
+        arrs[k] = a.astype(np.float64 if a.dtype == np.float64 or a.dtype.kind in "iub" else np.float32)
+    total = sum(a.nbytes for a in arrs.values())
+    for k, a in arrs.items():
+        if total > DUMP_BYTES and a.ndim > 0:
+            keep = max(1, a.shape[0] * DUMP_BYTES // total)
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(path, f"{k}.npy"), a)
+
+
 def render_block(name, r, ctx, steps, peak_tf, peak_src):
     """JSON sub-object of one render workload."""
     wl = WORKLOADS[name]
@@ -482,7 +508,11 @@ def main():
     ap.add_argument("--precision", default="exact", choices=["exact", "fast", "fp32"])
     ap.add_argument("--cpu-steps", type=int, default=6)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the primary workload's last timed step returned as DIR/<name>.npy (at most 64 MB)")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     ctx = Ctx(a)
     prim = a.workload
     is_mesh = prim == "mesh"
@@ -545,7 +575,8 @@ def main():
     if is_mesh:
         if clocks:
             clocks.start()
-        m = run_mesh(nm, ctx, a.steps, a.warmup, a.precision)
+        m = run_mesh(nm, ctx, a.steps, a.warmup, a.precision, keep=bool(a.dump_outputs))
+        outputs = m.pop("outputs", None)
         clk = clocks.stop() if clocks else None
         blk = mesh_block(m, a.steps)
         result.update({"value": blk["value"], "ms_per_step": blk["ms_per_step"], "clocks": clk, "gpu_launches": blk["gpu_launches"] * a.steps,
@@ -555,7 +586,8 @@ def main():
                                "api": "extract_geometry_sharded: the grid is generated on the device from three linspace tables "
                                       "(H2D) and the mesh stays on the device; only counts / statistics cross PCIe"}})
     else:
-        r = run_render(nm, prim, ctx, a.steps, a.warmup, a.precision, with_e2e=True, clocks=clocks)
+        r = run_render(nm, prim, ctx, a.steps, a.warmup, a.precision, with_e2e=True, clocks=clocks, keep=bool(a.dump_outputs))
+        outputs = r.pop("outputs", None)
         dev_ms, e2e_ms = ctx.max_over_ranks(r["dev_ms"], r["e2e_ms"])
         r["dev_ms"] = dev_ms
         blk = render_block(prim, r, ctx, a.steps, peak_tf, peak_src)
@@ -571,6 +603,8 @@ def main():
                        "gpu_launches": r["launches"], "roofline": blk["roofline"],
                        "e2e": {"value": r["rays"] / (e2e_ms * 1e-3), "unit": unit, "h2d_bytes_per_step": r["h2d"],
                                "d2h_bytes_per_step": r["d2h"], "api": r["e2e_api"]}})
+    if a.dump_outputs and ctx.rank == 0:
+        dump_outputs(a.dump_outputs, outputs)
 
     if not a.only:
         for name in ("lego", "fern", "buff"):

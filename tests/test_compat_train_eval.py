@@ -1,88 +1,22 @@
 """train_nerf.py / eval_nerf.py on the compat/ overlay (north_star: "so train_nerf.py, eval_nerf.py and mesh_nerf.py run
-unmodified").
-
-* Where the reference tree exists (the build container, no GPU): the reference's OWN scripts are executed, unmodified, on a
-  synthetic Blender-format dataset (tools/make_synthetic_blender.py): argument parsing, PathParser, the TensorBoard logger,
-  model construction, ModelCheckpoint / LoggerCallback, Trainer(...), fit -> setup -> the reference's Blender loader all run;
-  the first compute call (ray generation for the dataset) must end in the library's loud "needs a CUDA device" error — there
-  is no CPU path to fall into.
-* On the B200 box (no reference tree): the same call sequence is replayed against the overlay's modules with an in-memory
-  dataset of images rendered from the lego checkpoint: Trainer.fit (training_step on the fused loss+backward, optimiser /
-  scheduler steps, validation with image logging, ModelCheckpoint, resume), then the eval_nerf.py loop (batchify -> model.query
-  -> PSNR) on the checkpoint it wrote."""
+unmodified"): the scripts' call sequence is replayed against the overlay's modules with an in-memory dataset of images
+rendered from the lego checkpoint: Trainer.fit (training_step on the fused loss+backward, optimiser / scheduler steps,
+validation with image logging, ModelCheckpoint, resume), then the eval_nerf.py loop (batchify -> model.query -> PSNR) on
+the checkpoint it wrote."""
 import math
 import os
-import subprocess
 import sys
 
 import numpy as np
 import pytest
 import torch
-import yaml
 
 from conftest import ROOT
 
-REF = "/root/reference"
 sys.path.insert(0, os.path.join(ROOT, "tools"))
-needs_ref = pytest.mark.skipif(not os.path.isdir(REF + "/src"), reason="reference tree not on this machine")
 
 
-def run_script(script, args, cwd):
-    cmd = [sys.executable, os.path.join(ROOT, "compat", "run.py"), os.path.join(REF, "src", script)] + args
-    r = subprocess.run(cmd, capture_output=True, text=True, timeout=900, cwd=str(cwd))
-    return r.returncode, r.stdout + r.stderr
-
-
-@needs_ref
-@pytest.mark.skipif(torch.cuda.is_available(), reason="the GPU variant is test_reference_scripts_train_then_eval_on_gpu")
-def test_reference_train_script_runs_up_to_the_first_compute_call(tmp_path):
-    import make_synthetic_blender as M
-    cfg = M.make(str(tmp_path))
-    rc, out = run_script("train_nerf.py", ["--config", cfg], tmp_path)
-    assert "Logger initiated..." in out and "Finished reading from" in out, out[-3000:]      # PathParser, Trainer.fit -> setup -> loader
-    assert rc != 0 and "needs a CUDA device" in out, out[-3000:]
-    assert os.path.isdir(tmp_path / "logs" / "synthetic-lego" / "default" / "version_0" / "checkpoints")
-
-
-@needs_ref
-@pytest.mark.skipif(torch.cuda.is_available(), reason="the GPU variant is test_reference_scripts_train_then_eval_on_gpu")
-def test_reference_eval_script_runs_up_to_the_first_compute_call(tmp_path):
-    import make_synthetic_blender as M
-    cfg_path = M.make(str(tmp_path))
-    sys.path.insert(0, os.path.join(ROOT, "compat"))
-    try:
-        import models as ov
-        from nerfmeshes_b200.cfgnode import flatten_dict
-        cfg = yaml.safe_load(open(cfg_path))
-        model = ov.NeRFModel(cfg)
-        log_dir = tmp_path / "logs" / "synthetic-lego" / "default" / "version_0"
-        os.makedirs(log_dir / "checkpoints")
-        model.save_checkpoint(str(log_dir / "checkpoints" / "model_last.ckpt"), global_step=3)
-        yaml.dump({k: v for k, v in flatten_dict(cfg, sep=".").items()}, open(log_dir / "hparams.yaml", "w"))
-    finally:
-        sys.path.remove(os.path.join(ROOT, "compat"))
-        for m in [k for k in sys.modules if k.split(".")[0] in ("models", "nerf", "pytorch_lightning")]:
-            del sys.modules[m]
-    rc, out = run_script("eval_nerf.py", ["--log-checkpoint", str(log_dir), "--save-dir", str(tmp_path / "out"), "--save-images"], tmp_path)
-    assert "Loading model from" in out and "Finished reading from" in out, out[-3000:]        # checkpoint loaded, test split read
-    assert rc != 0 and "needs a CUDA device" in out, out[-3000:]
-
-
-@needs_ref
-@pytest.mark.gpu
-def test_reference_scripts_train_then_eval_on_gpu(tmp_path):
-    """A machine with both the reference tree and a B200: the unmodified scripts end to end."""
-    import make_synthetic_blender as M
-    cfg = M.make(str(tmp_path), render=True)
-    rc, out = run_script("train_nerf.py", ["--config", cfg], tmp_path)
-    assert rc == 0 and "Done!" in out, out[-3000:]
-    log_dir = tmp_path / "logs" / "synthetic-lego" / "default" / "version_0"
-    assert os.path.exists(log_dir / "checkpoints" / "model_last.ckpt") and os.path.exists(log_dir / "hparams.yaml")
-    rc, out = run_script("eval_nerf.py", ["--log-checkpoint", str(log_dir), "--save-dir", str(tmp_path / "out"), "--save-images"], tmp_path)
-    assert rc == 0 and "Dataset loss MSE" in out, out[-3000:]
-
-
-# ------------------------------------------------------------------------------------------------ GPU replay (no reference tree)
+# ------------------------------------------------------------------------------------------------ GPU replay
 class ImageDataset(torch.utils.data.Dataset):
     """What the reference's BlenderDataset yields per item (src/data/datasets.py:215-233): a dict of per-image tensors; the
     training split holds `num_random_rays` random rays of the image, the others the whole image."""

@@ -312,7 +312,7 @@ def test_full_size_image_properties(lego_model):
     assert float(err.max()) <= 6e-4 and float(err.quantile(0.99)) <= 1e-4, (float(err.max()), float(err.quantile(0.99)))
 
 
-def test_internal_chunking_is_invisible(lego_model):
+def test_internal_chunking_is_invisible(lego_model, tmp_path):
     """nm_render_rays splits very large batches internally; the split must not change a single bit."""
     import os
     import subprocess
@@ -325,7 +325,7 @@ def test_internal_chunking_is_invisible(lego_model):
     from conftest import ROOT
     outs = []
     for chunk, name in (("0", "a.pt"), ("700", "b.pt")):
-        path = os.path.join("/tmp", f"nm_chunk_{name}")
+        path = str(tmp_path / name)
         subprocess.run([sys.executable, "-c", code % (ROOT, ROOT), path], check=True, env=dict(os.environ, NM_CHUNK_RAYS=chunk), timeout=300)
         outs.append(torch.load(path))
     assert torch.equal(outs[0]["rgb"], outs[1]["rgb"]) and torch.equal(outs[0]["disp"], outs[1]["disp"])

@@ -233,14 +233,23 @@ def test_model_state_dict_matches_reference_checkpoint_keys():
     assert m.get_model() is m.model_fine and b.get_model() is b.model
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/pretrained"), reason="reference checkpoints not on this machine")
 def test_lightning_checkpoint_reader():
-    p = "/root/reference/pretrained/{}/default/version_0/checkpoints/model_last.ckpt"
-    m = nm.NeRFModel.load_from_checkpoint(p.format("colab-lego-nerf-high-res"))
+    """The shipped Lightning checkpoints (tests/golden/make_golden_ckpt.py: their 1-D tensors, hyper-parameters and BuFF
+    tree; the weight matrices are left out for size): every stored tensor lands in the module it names."""
+    p = os.path.join(ROOT, "tests", "golden", "ckpt_{}.ckpt")
+    m = nm.NeRFModel.load_from_checkpoint(p.format("lego_nerf"))
     z = load_npz("weights_lego_nerf.npz")
-    assert torch.equal(m.model_fine.layers_xyz[4].weight.data, z["fine.layers_xyz.4.weight"])
+    sd = m.state_dict()
+    n = 0
+    for prefix, key in (("model_coarse.", "coarse"), ("model_fine.", "fine")):
+        for k, v in net_weights(z, key).items():
+            if v.dim() == 1:
+                assert torch.equal(sd[prefix + k], v), k
+                n += 1
+    assert n == 24 and torch.equal(sd["sample_pdf.u"], z["sample_pdf_u"])
+    assert m.model_fine.layers_xyz[4].weight.shape == z["fine.layers_xyz.4.weight"].shape       # skip width from the hparams
     assert m.cfg.nerf.train.num_coarse == 64 and m.cfg.experiment.model == "NeRFModel"
-    b = nm.BuFFModel.load_from_checkpoint(p.format("buff-synthetic-lego"))
+    b = nm.BuFFModel.load_from_checkpoint(p.format("lego_buff"))
     assert torch.equal(b.tree.voxels, load_npz("weights_lego_buff.npz")["voxels"])
 
 

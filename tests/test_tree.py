@@ -86,18 +86,7 @@ def test_host_tree_construction_consolidate_and_schedule_match_reference():
 
 def test_checkpoint_tree_loads_into_host_classes_and_keeps_growing():
     import nerfmeshes_b200 as nm
-    p = "/root/reference/pretrained/colab-lego-buff/default/version_0/checkpoints"
-    ck = None
-    for base in ("/root/reference/pretrained",):
-        if os.path.isdir(base):
-            for d, _, files in os.walk(base):
-                for fn in files:
-                    if fn.endswith(".ckpt") and "buff" in d:
-                        ck = os.path.join(d, fn)
-    if ck is None:
-        import pytest
-        pytest.skip("reference checkpoints are not present on this box")
-    b = nm.BuFFModel.load_from_checkpoint(ck)
+    b = nm.BuFFModel.load_from_checkpoint(os.path.join(ROOT, "tests", "golden", "ckpt_lego_buff.ckpt"))
     assert isinstance(b.tree.root, T.Node) and len(b.tree.root.children) == b.tree.voxels.shape[0]
     n0 = b.tree.voxels.shape[0]
     b.tree.memm = torch.ones(n0)
