@@ -1,2 +1,2 @@
-def chamfer_distance(*a, **k):
-    raise NotImplementedError("pytorch3d is not available; chamfer evaluation is out of scope")
+"""pytorch3d.loss.chamfer_distance, backed by the CUDA nearest-neighbour kernel (nerfmeshes_b200.metrics)."""
+from nerfmeshes_b200.metrics import chamfer_distance  # noqa: F401

@@ -1,4 +1,2 @@
-class Meshes:
-    """Placeholder: only mesh_nerf.create_mesh (chamfer evaluation, off in every shipped config) would use it."""
-    def __init__(self, verts=None, faces=None):
-        self.verts, self.faces = verts, faces
+"""pytorch3d.structures.Meshes: the verts / faces batch that mesh_nerf.create_mesh builds (nerfmeshes_b200.metrics)."""
+from nerfmeshes_b200.metrics import Meshes  # noqa: F401

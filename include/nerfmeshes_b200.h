@@ -185,6 +185,23 @@ int nm_mc_emit(NmHandle h, const float* vol_dev, int nb, int ny, int nz, float i
 int nm_export_obj(const char* path, const float* verts_host, int64_t n_verts, const int32_t* faces_host, int64_t n_faces,
                   const float* diffuse_host, int64_t n_diffuse, const float* normals_host, int64_t n_normals);
 
+/* ---- mesh-quality metrics (the Chamfer metric of BaseModel.validation_epoch_end, src/models/model_base.py:82-102) ----- */
+/* The nearest-neighbour step of pytorch3d.loss.chamfer_distance (model_base.py:99): for each x_i of x (N,3) fp32, dist (N,)
+ * = min_j |x_i - y_j|^2 over y (M,3) fp32 and idx (N,) int32 = the argmin.  One pair's distance is
+ * ((dx*dx) + (dy*dy)) + (dz*dz), d = x - y, every operation rounded to nearest in fp32, no FMA contraction (a float32 numpy
+ * brute force reproduces it bit for bit); a tie goes to the lowest j, independent of how the work is split.  M >= 1,
+ * M < 2^31.  Exact brute force, N*M pair evaluations. */
+int nm_nearest(NmHandle h, const float* x_dev, int64_t N, const float* y_dev, int64_t M, float* dist_dev, int32_t* idx_dev,
+               void* stream);
+/* pytorch3d.ops.sample_points_from_meshes for one mesh (model_base.py:95-97): n points drawn on the surface of verts (V,3)
+ * fp32 / faces (F,3) int32 (indices in [0,V), not checked on the device), a face with probability proportional to its area
+ * 1/2|(v1-v0)x(v2-v0)| (with replacement), then p = w0 v0 + w1 v1 + w2 v2 with w0 = 1-sqrt(u), w1 = sqrt(u)(1-v),
+ * w2 = sqrt(u) v.  points (n,3); face_idx (n,) int32 and normals (n,3) (the sampled face's unit normal) may be NULL.  A mesh
+ * without faces or without area gives zero points and normals and face index -1.  Counter-based draws from `seed`: the
+ * same seed gives the same samples.  The area CDF (fp64, 8 bytes per face) lives in the handle's workspace. */
+int nm_mesh_sample(NmHandle h, const float* verts_dev, int64_t V, const int32_t* faces_dev, int64_t F, int64_t n, uint64_t seed,
+                   float* points_dev, int32_t* face_idx_dev_or_null, float* normals_dev_or_null, void* stream);
+
 /* ---- hot path, host buffers (what a reference-side caller holding CPU tensors binds) ------------------ */
 /* model.query(ray_batch) with host tensors (src/eval_nerf.py:62-69): copies H2D, renders, copies D2H, syncs. */
 int nm_query_host(NmHandle h, const float* origins_host, int o_stride, const float* dirs_host, int64_t R,

@@ -58,6 +58,8 @@ _SIGNATURES = {
     "nm_mc_count": (C.c_int, [_P, _P, _I, _I, _I, _F, _I, _I, _I, _I, _P, _P]),
     "nm_mc_emit": (C.c_int, [_P, _P, _I, _I, _I, _F, _I, _I, _I, _I, _L, _P, _P, _P, _P]),
     "nm_export_obj": (C.c_int, [C.c_char_p, _P, _L, _P, _L, _P, _L, _P, _L]),
+    "nm_nearest": (C.c_int, [_P, _P, _L, _P, _L, _P, _P, _P]),
+    "nm_mesh_sample": (C.c_int, [_P, _P, _L, _P, _L, _L, C.c_uint64, _P, _P, _P, _P]),
     "nm_query_host": (C.c_int, [_P, _P, _I, _P, _L, _P, _I, C.c_uint64, C.POINTER(NmRenderOut)]),
     "nm_render_image_host": (C.c_int, [_P, _P, _I, _I, _F, _I, _I, _I, _P, _I, C.c_uint64, C.POINTER(NmRenderOut)]),
     "nm_point_mlp_host": (C.c_int, [_P, _I, _P, _P, _L, _P, _I]),

@@ -24,6 +24,7 @@ SOURCES = {
     "nm_mlp_simt.cu": [],
     "nm_render.cu": ["-fmad=false"],
     "nm_mc.cu": ["-fmad=false"],
+    "nm_metrics.cu": ["-fmad=false"],
     "nm_train.cu": [],
     "nm_gemm_tc.cu": [],
     "nm_objwriter.cu": [],

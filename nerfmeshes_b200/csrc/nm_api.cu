@@ -65,6 +65,7 @@ struct NmHandle_t {
   // training (nm_train.cu): gradient accumulators per network + scratch
   Buf g_wt[2], g_bias[2], g_head[2], train_ws, dout, trans, tr_rgb[2], tr_drgb[2];
   bool grads_ready = false;
+  Buf metric_ws;                   // nearest-neighbour merge keys / area CDF of the surface sampler (nm_metrics.cu)
 };
 
 namespace {
@@ -471,7 +472,7 @@ int nm_destroy(NmHandle h) {
   for (Buf& b : h->stage_in) b.release();
   for (Buf& b : h->stage_out) b.release();
   for (int i = 0; i < 2; ++i) { h->g_wt[i].release(); h->g_bias[i].release(); h->g_head[i].release(); h->tr_rgb[i].release(); h->tr_drgb[i].release(); }
-  h->train_ws.release(); h->dout.release(); h->trans.release();
+  h->train_ws.release(); h->dout.release(); h->trans.release(); h->metric_ws.release();
   if (h->mc_ws_ptr) cudaFree(h->mc_ws_ptr);
   if (h->mc_ws2_ptr) cudaFree(h->mc_ws2_ptr);
   if (h->h_err) cudaFreeHost(h->h_err);
@@ -770,6 +771,29 @@ int nm_marching_cubes_emit(NmHandle h, const float* vol_dev, int nx, int ny, int
   const McShard s{vol_dev, nx, ny, nz, iso, 0, nx, 0, nx, (int)x_off};
   return mc_emit(s, h->mc_ws_ptr, h->mc_ws_bytes, &h->mc_ws2_ptr, &h->mc_ws2_bytes, 0, h->mc_counts[0], h->mc_counts[1], verts_dev,
                  normals_dev, faces_dev, (cudaStream_t)stream, &h->launches);
+}
+
+int nm_nearest(NmHandle h, const float* x_dev, int64_t N, const float* y_dev, int64_t M, float* dist_dev, int32_t* idx_dev,
+               void* stream) {
+  if (int e = bind_device(h)) return e;
+  NM_CHECK(N >= 0 && M >= 1 && M < (1ll << 31), "nearest: need N >= 0 and 1 <= M < 2^31 (got N=%lld, M=%lld)", (long long)N,
+           (long long)M);
+  NM_CHECK(N == 0 || (x_dev && y_dev && dist_dev && idx_dev), "null argument");
+  if (int e = h->metric_ws.ensure(nearest_ws_bytes(N, M, h->num_sms))) return e;
+  return launch_nearest(x_dev, N, y_dev, M, dist_dev, idx_dev, h->metric_ws.p, h->num_sms, (cudaStream_t)stream, &h->launches);
+}
+
+int nm_mesh_sample(NmHandle h, const float* verts_dev, int64_t V, const int32_t* faces_dev, int64_t F, int64_t n, uint64_t seed,
+                   float* points_dev, int32_t* face_idx_dev, float* normals_dev, void* stream) {
+  if (int e = bind_device(h)) return e;
+  NM_CHECK(V >= 0 && F >= 0 && n >= 0 && F < (1ll << 31), "mesh sample: bad sizes (V=%lld, F=%lld, n=%lld)", (long long)V,
+           (long long)F, (long long)n);
+  NM_CHECK(F == 0 || V > 0, "mesh sample: faces without vertices");
+  NM_CHECK(n == 0 || points_dev, "null output");
+  NM_CHECK(F == 0 || (verts_dev && faces_dev), "null mesh");
+  if (int e = h->metric_ws.ensure(mesh_sample_ws_bytes(F))) return e;
+  return launch_mesh_sample(verts_dev, faces_dev, F, n, seed, points_dev, face_idx_dev, normals_dev, h->metric_ws.p,
+                            (cudaStream_t)stream, &h->launches);
 }
 
 int nm_query_host(NmHandle h, const float* origins_host, int o_stride, const float* dirs_host, int64_t R,

@@ -205,5 +205,12 @@ struct McShard {
 int mc_count(const McShard& s, void** ws, size_t* ws_bytes, int64_t* counts_host, cudaStream_t st, int64_t* launches);
 int mc_emit(const McShard& s, void* ws, size_t ws_bytes, void** ws2, size_t* ws2_bytes, long long v_base, int64_t nv, int64_t nt,
             float* verts, float* normals, int32_t* faces, cudaStream_t st, int64_t* launches);
+// metrics (nm_metrics.cu): exact nearest neighbour and area-weighted surface sampling; callers size `ws` with the *_ws_bytes
+size_t nearest_ws_bytes(long long N, long long M, int num_sms);
+int launch_nearest(const float* x, long long N, const float* y, long long M, float* d, int* j, void* ws, int num_sms,
+                   cudaStream_t st, int64_t* launches);
+size_t mesh_sample_ws_bytes(long long F);
+int launch_mesh_sample(const float* verts, const int* faces, long long F, long long n, uint64_t seed, float* points, int* face_idx,
+                       float* normals, void* ws, cudaStream_t st, int64_t* launches);
 
 }  // namespace nm

@@ -11,13 +11,20 @@
 
 namespace nm {
 
-// counter-based uniform [0,1): splitmix64 of (seed, index).  Used only for perturb / noise (distributional parity).
-__device__ __forceinline__ float u01(uint64_t seed, uint64_t idx) {
+// counter-based random bits: splitmix64 of (seed, index)
+__device__ __forceinline__ uint64_t hash64(uint64_t seed, uint64_t idx) {
   uint64_t z = seed + 0x9E3779B97F4A7C15ull * (idx + 1);
   z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
   z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
-  z = z ^ (z >> 31);
-  return (float)(z >> 40) * (1.0f / 16777216.0f);
+  return z ^ (z >> 31);
+}
+// uniform [0,1) with 24 bits.  Used only for perturb / noise / surface sampling (distributional parity).
+__device__ __forceinline__ float u01(uint64_t seed, uint64_t idx) {
+  return (float)(hash64(seed, idx) >> 40) * (1.0f / 16777216.0f);
+}
+// uniform [0,1) with 53 bits, for draws that must resolve more than 2^24 outcomes (a face out of millions)
+__device__ __forceinline__ double u01_53(uint64_t seed, uint64_t idx) {
+  return (double)(hash64(seed, idx) >> 11) * (1.0 / 9007199254740992.0);
 }
 __device__ __forceinline__ float randn(uint64_t seed, uint64_t idx) {
   const float a = fmaxf(u01(seed, 2 * idx), 1e-7f), b = u01(seed, 2 * idx + 1);

@@ -438,6 +438,33 @@ class Engine:
                                         int(v_base), _ptr(verts), _ptr(normals), _ptr(faces), self._stream()))
         return verts, faces, normals
 
+    # ------------------------------------------------------------------ mesh-quality metrics (nm_metrics.cu)
+    def nearest(self, x: torch.Tensor, y: torch.Tensor):
+        """Exact nearest neighbour (nm_nearest): for x (N,3), y (M,3) CUDA fp32 on this device, returns dist (N,) fp32 =
+        min_j |x_i - y_j|^2 and idx (N,) int32 = the lowest j attaining it.  Inputs are not validated here
+        (nerfmeshes_b200.metrics does that)."""
+        x, y = _f32c(x, self.device), _f32c(y, self.device)
+        N, M = x.shape[0], y.shape[0]
+        dist = torch.empty((N,), dtype=torch.float32, device=self.device)
+        idx = torch.empty((N,), dtype=torch.int32, device=self.device)
+        if N:
+            L.check(self.lib.nm_nearest(self._h, _ptr(x), N, _ptr(y), M, _ptr(dist), _ptr(idx), self._stream()))
+        return dist, idx
+
+    def mesh_sample(self, verts: torch.Tensor, faces: torch.Tensor, n: int, seed: int, return_face=False, return_normals=False):
+        """Area-weighted surface sampling of one mesh (nm_mesh_sample): points (n,3) [, face index (n,) int32]
+        [, unit face normals (n,3)].  faces must index verts (checked by nerfmeshes_b200.metrics, not here)."""
+        v = _f32c(verts, self.device)
+        f = torch.as_tensor(faces).to(self.device, torch.int32).contiguous()
+        n = int(n)
+        pts = torch.empty((n, 3), dtype=torch.float32, device=self.device)
+        fi = torch.empty((n,), dtype=torch.int32, device=self.device) if return_face else None
+        nrm = torch.empty((n, 3), dtype=torch.float32, device=self.device) if return_normals else None
+        L.check(self.lib.nm_mesh_sample(self._h, _ptr(v), v.shape[0], _ptr(f), f.shape[0], n, int(seed) & 0xFFFFFFFFFFFFFFFF,
+                                        _ptr(pts), _ptr(fi), _ptr(nrm), self._stream()))
+        out = (pts,) + ((fi,) if return_face else ()) + ((nrm,) if return_normals else ())
+        return out if len(out) > 1 else pts
+
     # ------------------------------------------------------------------ introspection
     def kernel_flags(self):
         out = (C.c_int32 * 2)()

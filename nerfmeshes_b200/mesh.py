@@ -7,6 +7,17 @@ import torch
 from . import _lib as L
 
 
+def create_mesh(vertices, faces_idx):
+    """src/mesh_nerf.py:14-24: centre the vertices on their mean, divide by the largest absolute coordinate (the mesh then fits
+    the cube [-1,1]^3), and wrap the result in a one-mesh Meshes batch (nerfmeshes_b200.metrics)."""
+    from .metrics import Meshes
+    vertices = torch.as_tensor(vertices)
+    vertices = vertices - vertices.mean(0)
+    scale = vertices.abs().max(0)[0].max()
+    vertices = vertices / scale
+    return Meshes(verts=[vertices], faces=[torch.as_tensor(faces_idx)])
+
+
 def extract_radiance(model, args, device, nums, sigma_only=False, slab=None):
     """src/mesh_nerf.py:27-53.  Returns the (n0,n1,n2,4) numpy radiance grid like the reference, or — with
     sigma_only — the (n0,n1,n2) raw-density DEVICE tensor (the fast path extract_geometry uses; the reference
